@@ -2,10 +2,11 @@
 """bench.py — the BASELINE.json configs on B200, one JSON line (contract: DESIGN.md §Measurement).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload all|vitl14|knn|ivf|e2e|plumbing]
+                  [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`):
-  plumbing configs[0] ViT-B/32 clip_inference on 100 synthetic images + captions through the reference's own reader /
-                      runner / writer (baseline/_ref, unmodified) around the CUDA ClipMapper     -> samples/s
+  plumbing configs[0] ViT-B/32 clip_inference on 100 synthetic images + captions: the original project's reader /
+                      runner / writer job, replayed from its record, around the CUDA ClipMapper -> samples/s
   vitl14  configs[1]  ViT-L/14 image+text inference, synthetic 224^2, batch 1024 per GPU   -> pairs/s
   knn     configs[2]  brute-force cosine kNN, 100M x 768 fp16 rows per GPU, 1000 queries, top-40 -> queries/s
   ivf     configs[3]  IVF-Flat (nlist 65536, nprobe 16/64), rows range-sharded over the ranks, one all-gather -> queries/s
@@ -20,6 +21,9 @@ max over ranks); `e2e` = the same metric through the host-buffer API (H2D/D2H in
 `cpu_baseline` = the oracle port on the host cores on a bounded sample (rank 0, N=1 only);
 `parity_checked` = results of the timed configuration verified after the timed region (oracle as the checker).
 `--impl reference`: the CPU oracle port of the same workload on the host cores (bounded sample per step).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what each timed path returned in its last step as
+DIR/<workload>_<array>.npy (float32, ids as float64; a seeded row sample of an array over 4 MB, its row numbers in
+DIR/<workload>_<array>_rows.npy).  Inputs and weights are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -224,6 +228,7 @@ class Ctx:
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
         self.peaks = load_peaks()
+        self.dump_bytes = 0
         import clip_retrieval_b200 as m
 
         self.m = m
@@ -262,6 +267,41 @@ class Ctx:
     def sampler(self):
         return ClockSampler(self.local).start() if self.rank == 0 else None
 
+    def keep_outputs(self, workload, **arrays):
+        """--dump-outputs: rank 0 writes `arrays` (device tensors or numpy) as DIR/<workload>_<name>.npy."""
+        if self.args.dump_outputs and self.rank == 0:
+            self.dump_bytes += dump_outputs(self.args.dump_outputs, workload, arrays, DUMP_TOTAL_BYTES - self.dump_bytes)
+
+
+DUMP_ARRAY_BYTES = 4 << 20     # an array larger than this is cut to a seeded sample of its rows
+DUMP_TOTAL_BYTES = 64 << 20    # all arrays of one run, row numbers of the samples included
+
+
+def dump_outputs(folder, workload, arrays, budget):
+    """Writes `arrays` as float32 (ids and other integers as float64) .npy files in `folder`, each within
+    DUMP_ARRAY_BYTES and all of them within `budget` bytes; returns the bytes written."""
+    import numpy as np
+
+    os.makedirs(folder, exist_ok=True)
+    used = 0
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        a = np.atleast_1d(a.astype(np.float64 if a.dtype.kind in "iub" or a.dtype == np.float64 else np.float32))
+        base = os.path.join(folder, "%s_%s" % (workload, name))
+        cap = min(DUMP_ARRAY_BYTES, budget - used) - 2 * 256          # two .npy headers (128 bytes each as numpy writes them)
+        if a.nbytes > cap:
+            row_bytes = a.nbytes // a.shape[0] + 8                      # + its row number in <name>_rows.npy
+            keep = min(a.shape[0], cap // row_bytes)
+            if keep < 1:
+                raise SystemExit("--dump-outputs: %s_%s does not fit the %d bytes left of the dump" % (workload, name, budget - used))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            a = a[rows]
+            np.save(base + "_rows.npy", rows.astype(np.float64))
+            used += os.path.getsize(base + "_rows.npy")
+        np.save(base + ".npy", a)
+        used += os.path.getsize(base + ".npy")
+    return used
+
 
 def synth_tokens(torch, n, arch, gen, lo=3, hi=None):
     hi = hi or (arch.context_length - 2)
@@ -290,9 +330,10 @@ def wl_vitl14(ctx):
     tok_host = synth_tokens(torch, B, arch, g).pin_memory()
     px_dev, tok_dev = px_host.to(ctx.dev), tok_host.to(ctx.dev)
 
+    last = [None]
+
     def step_device():
-        model.embed_image_device(px_dev)
-        model.embed_text_device(tok_dev)
+        last[0] = (model.embed_image_device(px_dev), model.embed_text_device(tok_dev))
 
     for _ in range(W):
         step_device()
@@ -300,6 +341,8 @@ def wl_vitl14(ctx):
     launches0 = m.launch_count()
     ms_per_step = ctx.timed(step_device, K)                  # the timed region: no per-kernel events inside
     launches = m.launch_count() - launches0
+    ctx.keep_outputs("vitl14", image_embs=last[0][0], text_embs=last[0][1])
+    last[0] = None
     # per-kernel-class device time: a second pass of the same K steps with CUDA events around every kernel
     model.set_profiling(True)
     for _ in range(K):
@@ -451,13 +494,20 @@ def wl_knn(ctx):
     sh = m.ShardedIndex(idx, device=ctx.dev)
     q = synth_rows(nq, d, m.SynthSpec(seed=4321), dtype="float32", device=ctx.local)
     q1 = q[:1].contiguous()
-    Wk, Kk = max(1, min(args.warmup, 2)), max(1, args.knn_steps)
+    Wk, Kk = max(1, min(args.warmup, 2)), args.steps
     for _ in range(Wk):
         sh.search_device(q, k)
     sampler = ctx.sampler()
     launches0 = m.launch_count()
-    ms = ctx.timed(lambda: sh.search_device(q, k), Kk)
+    last = [None]
+
+    def step():
+        last[0] = sh.search_device(q, k)
+
+    ms = ctx.timed(step, Kk)
     launches = m.launch_count() - launches0
+    ctx.keep_outputs("knn", D=last[0][0], I=last[0][1])
+    last[0] = None
     s_ms, s_n = idx.last_scan_ms()
     fallbacks = idx.last_hi_only_fallbacks()
     # serving shape: one query at a time (clip_back.py:362 issues nq=1)
@@ -667,14 +717,21 @@ def wl_ivf(ctx, d=768):
     sampler = ctx.sampler()
     per = {}
     launches = 0
-    Kk = max(2, args.knn_steps)
+    Kk = args.steps
     for nprobe in (16, 64):
         idx.nprobe = nprobe
         for _ in range(2):
             sh.search_device(q, k)
         l0 = m.launch_count()
-        ms = ctx.timed(lambda: sh.search_device(q, k), Kk)
+        last = [None]
+
+        def step():
+            last[0] = sh.search_device(q, k)
+
+        ms = ctx.timed(step, Kk)
         launches += m.launch_count() - l0
+        ctx.keep_outputs("ivf", **{"nprobe%d_D" % nprobe: last[0][0], "nprobe%d_I" % nprobe: last[0][1]})
+        del last
         s_ms, s_n = idx.last_scan_ms()
         for _ in range(3):
             sh.search_device(q1, k)
@@ -787,13 +844,20 @@ def wl_e2e(ctx):
     launches = m.launch_count() - l0
     lat_ms = np.array(lat) * 1e3
     # device-resident throughput: batches of 64 queries, embed + search, results stay on the device
+    last = []
+
     def step_dev():
+        last.clear()
         for s in range(0, nreq - 63, 64):
             qv = model.embed_text_device(toks_dev[s:s + 64], dtype=torch.float32)
-            sh.search_device(qv, k)
+            last.append((qv,) + tuple(sh.search_device(qv, k)))
     step_dev()
     nb = len(range(0, nreq - 63, 64)) * 64
-    ms_dev = ctx.timed(step_dev, 3)
+    ms_dev = ctx.timed(step_dev, args.steps)
+    if last:
+        ctx.keep_outputs("e2e", query_embs=torch.cat([x[0] for x in last]), D=torch.cat([x[1] for x in last]),
+                         I=torch.cat([x[2] for x in last]))
+    last.clear()
     # closed loop through the micro-batching front: `conc` client threads, each waits for its answer before the next
     conc = 64
     mb = m.MicroBatcher(model, sh if ctx.world == 1 else idx, max_batch=64, max_wait_ms=0.3, k=k)
@@ -863,7 +927,7 @@ def wl_e2e(ctx):
     p50 = float(np.percentile(lat_ms, 50))
     out = {
         "metric": "clip_back query path queries/s (ViT-H/14 text -> embed -> IVF-Flat kNN over %d x %d rows per GPU -> ids)" % (rows, d),
-        "value": nb / (ms_dev / 1e3), "unit": "queries/s", "n_gpus": ctx.world, "steps": 3, "warmup": 1,
+        "value": nb / (ms_dev / 1e3), "unit": "queries/s", "n_gpus": ctx.world, "steps": args.steps, "warmup": 1,
         "ms_per_step": ms_dev, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "baseline_note": "README.md:433-435: reference averages 18.6 ms text embed + 26.7 ms knn on its CPU/A100 setup",
         "dtype": "bf16 text tower (fp32 accumulate), f16 rows / f32 query search", "data": "synthetic",
@@ -934,19 +998,9 @@ def cpu_baseline_e2e(ctx, arch, d, k, nprobe, rows_gpu, nlist_gpu, nquery=8):
 
 # ---- the B200 arm ---------------------------------------------------------------------------------------------
 # ---- configs[0]: the clip_inference plumbing (reference reader -> runner -> mapper -> writer) -------------------
-REF_INFERENCE = os.path.join(ROOT, "baseline", "_ref", "clip_retrieval", "clip_inference")
-
-
-def ref_inference_module(name):
-    """reader.py / runner.py / writer.py of the UNMODIFIED reference install under baseline/_ref, loaded by file path
-    (the package's __init__ imports flask/faiss/all_clip, which are not installable offline; these three files only
-    need torch, PIL, fsspec and pyarrow)."""
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(REF_INFERENCE, name + ".py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+# What the original project's FilesReader -> Runner -> NumpyWriter did over make_plumbing_dataset()'s files, recorded by
+# tests/golden/make_reference_golden.py: its code cannot be installed offline, so its job is replayed from this record.
+RUNNER_TRACE = os.path.join(ROOT, "tests", "golden", "reference_runner_trace.json")
 
 
 def hashed_tokenizer(texts, context_length=77, vocab=49408):
@@ -978,42 +1032,72 @@ def make_plumbing_dataset(folder, n, seed=0):
             f.write("a photo of object %d" % i)
 
 
+def load_runner_trace(n, parts, batch_size):
+    with open(RUNNER_TRACE) as f:
+        for t in json.load(f):
+            if (t["samples"], t["partitions"], t["batch_size"]) == (n, parts, batch_size):
+                return t
+    raise ValueError("no recorded clip_inference job with %d samples, %d partitions, batch %d in %s"
+                     % (n, parts, batch_size, RUNNER_TRACE))
+
+
+def _batch_fields(batch):
+    import torch
+
+    return {k: [str(v.dtype), list(v.shape)] if torch.is_tensor(v) else type(v).__name__ for k, v in sorted(batch.items())}
+
+
 def run_reference_runner(src, out_root, mapper, preprocess, tokenizer, parts=2, batch_size=32):
-    """One clip_inference job through the reference's own FilesReader, Runner and NumpyWriter (runner.py:17-62):
-    the reference keys files by path INCLUDING the extension (reader.py:17-32), so image and caption keys never
-    intersect and a folder job is one pass over the images and one over the captions (as its own tests do,
-    test_reader.py:39).  `mapper` is the ClipMapper-contract callable under test.  Returns seconds inside mapper()."""
-    reader, runner, writer = ref_inference_module("reader"), ref_inference_module("runner"), ref_inference_module("writer")
-    spent = [0.0]
+    """One clip_inference job as the original project's own FilesReader, Runner and NumpyWriter run it
+    (runner.py:17-62), replayed from RUNNER_TRACE over make_plumbing_dataset()'s `NNNN.png` / `NNNN.txt` in `src`:
+    the batches its reader yielded (checked field by field: keys, tensor dtypes and shapes, sample files), in the
+    order its Runner handed them to the mapper, and the .npy shards its writer left (checked against the recorded
+    path, dtype, rows and sample order; the metadata parquet files it also writes are not reproduced).  The original
+    keys files by path INCLUDING the extension (reader.py:17-32), so image and caption keys never intersect and a
+    folder job is one pass over the images and one over the captions (as its own tests do, test_reader.py:39).
+    `mapper(batch, img, txt)` is the ClipMapper-contract callable under test.  Returns seconds inside mapper()."""
+    import numpy as np
+    import torch
+    from PIL import Image
 
-    class Logger:
-        def start(self): pass
-        def end(self): pass
-        def __call__(self, stats): pass
-
-    for modality in ("image", "text"):
-        img, txt = modality == "image", modality == "text"
-
-        def call(batch, img=img, txt=txt):
+    n = sum(1 for f in os.listdir(src) if f.endswith(".png"))
+    trace = load_runner_trace(n, parts, batch_size)
+    spent = 0.0
+    rows = {}
+    for run in trace["runs"]:
+        img = run["modality"] == "image"
+        embs, samples = [], []
+        for b in run["batches"]:
+            if img:
+                files = [os.path.join(src, f) for f in b["image_filename"]]
+                batch = {"image_filename": files, "image_tensor": torch.stack([preprocess(Image.open(f)) for f in files])}
+            else:
+                texts = []
+                for i in b["samples"]:
+                    with open(os.path.join(src, "%04d.txt" % i)) as f:
+                        texts.append(f.read())
+                if texts != b["text"]:
+                    raise ValueError("captions in %s differ from the recorded job" % src)
+                batch = {"text": texts, "text_tokens": tokenizer(texts)}
+            if _batch_fields(batch) != b["fields"]:
+                raise ValueError("batch %r differs from the recorded reader batch %r" % (_batch_fields(batch), b["fields"]))
             t0 = time.perf_counter()
-            r = mapper(batch, img, txt)
-            spent[0] += time.perf_counter() - t0
-            return r
-
-        out = os.path.join(out_root, "out_" + modality)
-        run = runner.Runner(
-            reader_builder=lambda sampler, img=img, txt=txt: reader.FilesReader(
-                sampler, preprocess, tokenizer, src, batch_size, 0, enable_text=txt, enable_image=img, enable_metadata=False),
-            mapper_builder=lambda call=call: call,
-            writer_builder=lambda i, out=out, img=img, txt=txt: writer.NumpyWriter(
-                partition_id=i, output_folder=out, enable_text=txt, enable_image=img, enable_metadata=False,
-                output_partition_count=parts),
-            logger_builder=lambda i: Logger(),
-            output_partition_count=parts,
-        )
-        for i in range(parts):
-            run(i)
-    return spent[0]
+            r = mapper(batch, img, not img)
+            spent += time.perf_counter() - t0
+            embs.append(r["image_embs"] if img else r["text_embs"])
+            samples += b["samples"]
+        rows[(run["modality"], tuple(samples))] = np.concatenate(embs)
+    for f in trace["files"]:
+        if not f["path"].endswith(".npy"):
+            continue
+        a = rows.pop((f["path"].split("/")[0][len("out_"):], tuple(f["samples"])))
+        if str(a.dtype) != f["dtype"] or a.shape[0] != f["shape"][0]:
+            raise ValueError("shard %s: %s %r, the recorded writer left %s %r" % (f["path"], a.dtype, a.shape, f["dtype"], f["shape"]))
+        path = os.path.join(out_root, f["path"])
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        np.save(path, a)
+    assert not rows, "mapper output not written by the recorded writer: %r" % list(rows)
+    return spent
 
 
 def read_plumbing_output(out_root):
@@ -1026,8 +1110,9 @@ def read_plumbing_output(out_root):
 
 
 def wl_plumbing(ctx):
-    """BASELINE configs[0]: ViT-B/32 clip_inference on 100 synthetic images + captions — the reference's reader,
-    runner and writer, unmodified, around the CUDA `ClipMapper`; the CPU arm is the same job around the fp32 oracle."""
+    """BASELINE configs[0]: ViT-B/32 clip_inference on 100 synthetic images + captions — the original project's
+    reader / runner / writer job (replayed from its record) around the CUDA `ClipMapper`; the CPU arm is the same job
+    around the fp32 oracle."""
     import shutil
     import tempfile
 
@@ -1038,13 +1123,9 @@ def wl_plumbing(ctx):
     n, parts, bs = 100, 2, 32
     base = {"metric": "ViT-B/32 clip_inference samples/s (image + caption files -> fp16 .npy shards)", "unit": "samples/s",
             "n_gpus": ctx.world, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
-            "config": {"workload": "ViT-B/32 clip_inference on %d synthetic images + captions per GPU through the reference's own FilesReader / "
-                                   "Runner / NumpyWriter (baseline/_ref, unmodified), batch %d, %d output partitions (BASELINE configs[0])"
-                                   % (n, bs, parts)}}
-    if not os.path.isdir(REF_INFERENCE):
-        base.update({"unavailable": "baseline/_ref (the reference install, made by __graft_entry__.build() where /root/reference exists) "
-                                    "is not in this tree", "parity_checked": None})
-        return base
+            "config": {"workload": "ViT-B/32 clip_inference on %d synthetic images + captions per GPU: the batches and .npy shards of the "
+                                   "original project's FilesReader / Runner / NumpyWriter job (tests/golden/reference_runner_trace.json), "
+                                   "batch %d, %d output partitions (BASELINE configs[0])" % (n, bs, parts)}}
     tmp = tempfile.mkdtemp(prefix="b200clip_plumbing_%d_" % ctx.rank)
     try:
         src = os.path.join(tmp, "images")
@@ -1060,7 +1141,7 @@ def wl_plumbing(ctx):
             mapper.enable_image, mapper.enable_text = img, txt
             return mapper(batch)
 
-        steps, times, inside = max(1, min(ctx.args.steps, 3)), [], []
+        steps, times, inside = ctx.args.steps, [], []
         launches0 = None
         for it in range(1 + steps):                                      # one warm-up job, then `steps` timed jobs
             out = os.path.join(tmp, "gpu_%d" % it)
@@ -1076,6 +1157,9 @@ def wl_plumbing(ctx):
                 inside.append(sec)
         launches = (m.launch_count() - launches0) // steps
         t_job = statistics.median(times)
+        if ctx.args.dump_outputs:
+            img_l, txt_l = read_plumbing_output(os.path.join(tmp, "gpu_%d" % steps))
+            ctx.keep_outputs("plumbing", image_embs=np.concatenate(img_l), text_embs=np.concatenate(txt_l))
         img_g, txt_g = read_plumbing_output(os.path.join(tmp, "gpu_1"))
         ok_layout = (len(img_g) == parts and len(txt_g) == parts
                      and all(a.dtype == np.float16 and a.shape == (n // parts, arch.embed_dim) for a in img_g + txt_g))
@@ -1086,8 +1170,8 @@ def wl_plumbing(ctx):
                             "h2d_bytes_per_step": n * (3 * arch.image_size ** 2 * 4 + arch.context_length * 8),
                             "d2h_bytes_per_step": 2 * n * arch.embed_dim * 2},
                     "mapper_ms_per_step": 1e3 * statistics.median(inside),
-                    "note": "host-bound by design: PNG decode + torchvision Resize/CenterCrop run in the reference's DataLoader "
-                            "(num_workers 0) on one host thread; `mapper_ms_per_step` is the part this engine replaces "
+                    "note": "host-bound by design: PNG decode + torchvision Resize/CenterCrop run on one host thread, as in the "
+                            "original's DataLoader (num_workers 0); `mapper_ms_per_step` is the part this engine replaces "
                             "(H2D, both towers, normalise, fp16, D2H for %d images and %d captions)" % (n, n)})
         res["roofline"] = None
         if ctx.rank == 0 and not ctx.args.no_cpu:
@@ -1110,7 +1194,7 @@ def wl_plumbing(ctx):
             dt_cpu = time.perf_counter() - t0
             res["cpu_baseline"] = {"value": n / dt_cpu, "unit": "samples/s", "cores": cores, "kind": "port",
                                    "mapper_ms_per_step": 1e3 * sec_cpu,
-                                   "sample": "the same %d-sample job once, same reference reader/runner/writer, mapper = fp32 oracle/clip_ref.py "
+                                   "sample": "the same %d-sample job once, same recorded reader/runner/writer job, mapper = fp32 oracle/clip_ref.py "
                                              "with %d torch threads (the reference's own mapper needs all_clip/open_clip, not installable)"
                                              % (n, cores)}
             img_c, txt_c = read_plumbing_output(os.path.join(tmp, "cpu"))
@@ -1161,18 +1245,14 @@ def run_reference(args):
     if rank != 0:
         return
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    K, W = max(1, min(args.steps, 3)), 1
+    K, W = args.steps, 1
     cores = physical_cores()
     n = max(2, min(args.cpu_sample, 64))
-    vals, secs = [], []
-    t_all = time.perf_counter()
+    vals = []
     cpu_embed_sample("ViT-L/14", min(4, n), cores, budget_s=20.0)            # warm-up step
     for _ in range(K):
         v, done, dt = cpu_embed_sample("ViT-L/14", n, cores, budget_s=60.0)
         vals.append(v)
-        secs.append(dt)
-        if time.perf_counter() - t_all > 200:
-            break
     value = statistics.median(vals)
     cb = {"value": value, "unit": "pairs/s", "cores": cores, "kind": "port",
           "sample": "median of %d steps of %d image+text pairs (chunks of 16), fp32 oracle/clip_ref.py, torch %d threads (physical cores); "
@@ -1230,12 +1310,15 @@ def main():
     ap.add_argument("--no-plumbing", action="store_true")
     ap.add_argument("--knn-rows", type=int, default=100_000_000)
     ap.add_argument("--knn-nq", type=int, default=1000)
-    ap.add_argument("--knn-steps", type=int, default=2)
     ap.add_argument("--ivf-rows", type=int, default=100_000_000)
     ap.add_argument("--ivf-nlist", type=int, default=65536)
     ap.add_argument("--e2e-rows", type=int, default=75_000_000)
     ap.add_argument("--e2e-queries", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs of every workload run as DIR/<workload>_<array>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1 (every workload times exactly --steps steps)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -21,6 +21,35 @@ def test_reference_arm_prints_one_json_line():
     assert j["e2e"]["h2d_bytes_per_step"] == 0 and j["e2e"]["d2h_bytes_per_step"] == 0
     for key in ("metric", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "dtype", "data", "config"):
         assert key in j
+    assert j["steps"] == 1
+
+
+def test_steps_below_one_are_rejected():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr and r.stdout.strip() == ""
+
+
+def test_dump_outputs_stays_within_its_budget(tmp_path):
+    """--dump-outputs: float32 / float64 files, a seeded row sample (with its row numbers) of an array over the
+    per-array cap, 1-D arrays included, and never more bytes on disk than the budget it is given."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    big = np.random.default_rng(1).standard_normal((4096, 1024)).astype(np.float16)
+    ids = np.arange(3_000_000, dtype=np.int64)
+    used = bench.dump_outputs(str(tmp_path), "w", {"embs": big, "I": ids}, 6 << 20)
+    files = {f: os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert used == sum(files.values()) <= 6 << 20
+    e, rows = np.load(tmp_path / "w_embs.npy"), np.load(tmp_path / "w_embs_rows.npy")
+    assert e.dtype == np.float32 and rows.dtype == np.float64 and np.array_equal(e, big[rows.astype(np.int64)].astype(np.float32))
+    i, irows = np.load(tmp_path / "w_I.npy"), np.load(tmp_path / "w_I_rows.npy")
+    assert i.dtype == np.float64 and np.array_equal(i, irows)
+    again = tmp_path / "again"
+    bench.dump_outputs(str(again), "w", {"embs": big}, 6 << 20)
+    assert np.array_equal(np.load(again / "w_embs_rows.npy"), rows)      # the same rows from run to run
 
 
 def test_reference_arm_other_ranks_exit_quietly():
@@ -32,10 +61,10 @@ def test_reference_arm_other_ranks_exit_quietly():
 
 def test_plumbing_helpers_drive_the_reference_runner(tmp_path):
     """configs[0] helpers of bench.py on the CPU: the synthetic tokenizer ends every caption with the largest id (the
-    text tower pools at argmax), and a ClipMapper-contract callable driven by the reference's own Runner (baseline/_ref)
-    produces the writer's shard layout in the sampler's order."""
+    text tower pools at argmax), and a ClipMapper-contract callable driven through bench's replay of the original
+    project's own Runner job (tests/golden/reference_runner_trace.json) produces the writer's shard layout in the
+    sampler's order."""
     import numpy as np
-    import pytest
     import torch
 
     sys.path.insert(0, ROOT)
@@ -44,8 +73,6 @@ def test_plumbing_helpers_drive_the_reference_runner(tmp_path):
     tok = bench.hashed_tokenizer(["a photo of object 3", "", "x " * 200])
     assert tok.shape == (3, 77) and tok.dtype == torch.int64
     assert all(int(row.argmax()) == int((row != 0).sum()) - 1 and int(row.max()) == 49407 and int(row[0]) == 49406 for row in tok)
-    if not os.path.isdir(bench.REF_INFERENCE):
-        pytest.skip("baseline/_ref (reference install) not in this tree")
     from clip_retrieval_b200.model import make_preprocess
 
     n, parts, bs, d = 10, 2, 4, 16

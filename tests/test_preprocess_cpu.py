@@ -1,10 +1,8 @@
 """Pins the preprocess oracle (oracle/preprocess_ref.py): against Pillow + torchvision running here,
-against the committed golden derived from the reference's test_tensors fixtures, and — when
-/root/reference is present (build container) — against those fixtures directly."""
-import glob
+and against the reference's test_tensors fixtures (their sha256 in the committed golden), both from the
+stored decoded pixels and from the reference's own test images (tests/golden/reference_images)."""
 import hashlib
 import os
-import pickle
 
 import numpy as np
 import pytest
@@ -12,7 +10,7 @@ import pytest
 from oracle import preprocess_ref as P
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "preprocess_ref.npz")
-REF = "/root/reference/tests/test_clip_inference"
+REF_IMAGES = os.path.join(os.path.dirname(__file__), "golden", "reference_images")
 
 
 def _torchvision_transform(n_px):
@@ -54,17 +52,17 @@ def test_oracle_matches_committed_reference_golden():
     assert n == 4
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
 def test_oracle_matches_reference_fixtures():
+    """The reference's 7 test images, decoded with Pillow, against the sha256 of the float32 tensors its
+    preprocess produced for them (test_tensors/*.pkl; tests/golden/make_preprocess_golden.py)."""
     from PIL import Image
+    g = np.load(GOLD)
     seen = 0
-    for f in sorted(glob.glob(REF + "/test_tensors/*.pkl")):
-        with open(f, "rb") as fh:
-            o = pickle.load(fh)
-        for name, t in zip(o["image_filename"], o["image_tensor"]):
-            px = np.asarray(Image.open(f"{REF}/test_images/{name}.jpg").convert("RGB"))
-            assert np.array_equal(P.preprocess(px), t.numpy()), name
-            seen += 1
+    for name in g["names"]:
+        px = np.asarray(Image.open(os.path.join(REF_IMAGES, f"{name}.jpg")).convert("RGB"))
+        got = P.preprocess(px)
+        assert hashlib.sha256(got.tobytes()).digest() == g[f"sha256_{name}"].tobytes(), name
+        seen += 1
     assert seen == 7
 
 

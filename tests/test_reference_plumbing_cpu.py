@@ -1,32 +1,20 @@
 """BASELINE.json configs[0] — "ViT-B/32 clip_inference on 100 synthetic 224^2 images + captions, CPU ref
-(plumbing)" — run through the REFERENCE'S OWN reader, runner and writer (importable by file path in the
-build container: reader.py / runner.py / writer.py only need torch, PIL, fsspec, pyarrow) with the
-reference's own `ClipMapper.__call__` (extracted with ast; its `all_clip` model is replaced by the oracle's
-ViT-B/32 encoders, seeded weights).  What it pins, on the reference's code:
-  * the `preprocess` object `clip_retrieval_b200.load_clip` returns drops into `FilesReader`;
-  * the batch dict the reader yields is the one the mapper contract (SURVEY §8b B1) describes;
+(plumbing)" — bench.run_reference_runner's replay of what the ORIGINAL project's own reader, runner and
+writer did with this dataset (tests/golden/reference_runner_trace.json, recorded by
+tests/golden/make_reference_golden.py), with the oracle's ViT-B/32 encoders (seeded weights) behind the mapper
+glue that tests/test_oracle_cpu.py pins on the original `ClipMapper.__call__`.  What it pins:
+  * the `preprocess` object `clip_retrieval_b200.load_clip` returns builds the batches the original `FilesReader`
+    yielded (fields, dtypes, shapes);
+  * the batch dict is the one the mapper contract (SURVEY §8b B1) describes;
   * the writer's shard layout (`img_emb/img_emb_{i}.npy`, fp16, partition order) is what
     `clip_retrieval_b200.load_index` enumerates, row for row.
 The GPU mapper itself is tested against the same oracle in tests/test_embed_gpu.py."""
-import ast
-import importlib.util
 import os
-import textwrap
-import types
 
 import numpy as np
-import pytest
 import torch
 
-REF = "/root/reference/clip_retrieval/clip_inference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
-
-
-def _ref_module(name):
-    spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(REF, name + ".py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+import bench
 
 
 def _synthetic_tokenizer(texts):
@@ -46,7 +34,6 @@ def test_config0_plumbing_reference_reader_runner_writer(tmp_path):
     from clip_retrieval_b200.index import list_embedding_shards
     from clip_retrieval_b200.model import make_preprocess
 
-    reader, runner, writer = _ref_module("reader"), _ref_module("runner"), _ref_module("writer")
     n = 100
     rng = np.random.default_rng(0)
     src = tmp_path / "images"
@@ -58,50 +45,26 @@ def test_config0_plumbing_reference_reader_runner_writer(tmp_path):
 
     cfg = clip_ref.CONFIGS["ViT-B/32"]
     sd = clip_ref.make_state_dict(cfg, seed=0)
-    msrc = open(os.path.join(REF, "mapper.py")).read()
-    cls = next(x for x in ast.parse(msrc).body if isinstance(x, ast.ClassDef) and x.name == "ClipMapper")
-    call = next(x for x in cls.body if isinstance(x, ast.FunctionDef) and x.name == "__call__")
-    ns = {"torch": torch, "np": np}
-    exec(textwrap.dedent(ast.get_source_segment(msrc, call)), ns)
     seen = {"image": 0, "text": 0}
 
-    class Logger:
-        def start(self): pass
-        def end(self): pass
-        def __call__(self, stats): assert stats["sample_count"] > 0
+    def mapper(batch, img, txt):
+        if img:
+            assert batch["image_tensor"].dtype == torch.float32 and tuple(batch["image_tensor"].shape[1:]) == (3, 224, 224)
+            assert len(batch["image_filename"]) == batch["image_tensor"].shape[0]
+            seen["image"] += batch["image_tensor"].shape[0]
+        else:
+            assert batch["text_tokens"].shape[1] == 77 and len(batch["text"]) == batch["text_tokens"].shape[0]
+            seen["text"] += batch["text_tokens"].shape[0]
+        return {"image_embs": clip_ref.mapper_image(sd, cfg, batch["image_tensor"]) if img else None,
+                "text_embs": clip_ref.mapper_text(sd, cfg, batch["text_tokens"]) if txt else None,
+                "image_filename": batch["image_filename"] if img else None, "text": batch["text"] if txt else None,
+                "metadata": None}
 
-    # The reference's FilesReader keys files by relative path INCLUDING the extension (reader.py:17-32), so
-    # image and caption keys never intersect; its own tests read images only (test_reader.py:39).  Same here:
-    # one pass over the images, one over the captions.
+    # The original FilesReader keys files by relative path INCLUDING the extension (reader.py:17-32), so image and
+    # caption keys never intersect; its own tests read images only (test_reader.py:39).  The recorded job is one pass
+    # over the images and one over the captions, two output partitions each.
     parts = 2
-    for modality in ("image", "text"):
-        img, txt = modality == "image", modality == "text"
-        me = types.SimpleNamespace(enable_image=img, enable_text=txt, enable_metadata=False, use_mclip=False, device="cpu",
-                                   model_img=lambda x: clip_ref.encode_image(sd, cfg, x),
-                                   model_txt=lambda x: clip_ref.encode_text(sd, cfg, x))
-
-        def mapper(batch, me=me, img=img):
-            if img:
-                assert batch["image_tensor"].dtype == torch.float32 and tuple(batch["image_tensor"].shape[1:]) == (3, 224, 224)
-                assert len(batch["image_filename"]) == batch["image_tensor"].shape[0]
-                seen["image"] += batch["image_tensor"].shape[0]
-            else:
-                assert batch["text_tokens"].shape[1] == 77 and len(batch["text"]) == batch["text_tokens"].shape[0]
-                seen["text"] += batch["text_tokens"].shape[0]
-            return ns["__call__"](me, batch)
-
-        out = tmp_path / ("out_" + modality)
-        run = runner.Runner(
-            reader_builder=lambda sampler: reader.FilesReader(sampler, make_preprocess(224), _synthetic_tokenizer, str(src), 32, 0,
-                                                              enable_text=txt, enable_image=img, enable_metadata=False),
-            mapper_builder=lambda: mapper,
-            writer_builder=lambda i: writer.NumpyWriter(partition_id=i, output_folder=str(out), enable_text=txt, enable_image=img,
-                                                        enable_metadata=False, output_partition_count=parts),
-            logger_builder=lambda i: Logger(),
-            output_partition_count=parts,
-        )
-        for i in range(parts):
-            run(i)
+    bench.run_reference_runner(str(src), str(tmp_path), mapper, make_preprocess(224), _synthetic_tokenizer, parts, 32)
     assert seen == {"image": n, "text": n}
 
     shards = list_embedding_shards(str(tmp_path / "out_image" / "img_emb"))

@@ -1,8 +1,9 @@
-"""BASELINE.json configs[0] on the GPU: the reference's OWN FilesReader, Runner and NumpyWriter — the unmodified
-install under baseline/_ref, which travels to the GPU box (/root/reference does not) — around the CUDA `ClipMapper`
-(clip_retrieval/clip_inference/runner.py:27-62 calls `mapper(batch)` and hands the dict to `writer`; worker.py:52-117
-builds exactly these objects).  The written shards are compared row for row with the fp32 oracle mapper applied to
-the same files in the partition order `runner.Sampler` defines, and loaded back through `load_index`."""
+"""BASELINE.json configs[0] on the GPU: the CUDA `ClipMapper` fed the batches the original project's own FilesReader,
+Runner and NumpyWriter formed over bench.py's dataset, its output written to the files that writer left — bench's
+replay of tests/golden/reference_runner_trace.json (clip_retrieval/clip_inference/runner.py:27-62 calls `mapper(batch)` and hands
+the dict to `writer`; worker.py:52-117 builds exactly these objects).  The written shards are compared row for row with
+the fp32 oracle mapper applied to the same files in the partition order `runner.Sampler` defines, and loaded back
+through `load_index`."""
 import os
 
 import numpy as np
@@ -11,8 +12,7 @@ import pytest
 import bench
 from oracle import clip_ref
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isdir(bench.REF_INFERENCE), reason="baseline/_ref (reference install) not in this tree")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.timeout(600)
